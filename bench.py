@@ -47,7 +47,31 @@ def parse():
     ap.add_argument("--graph", action="store_true", help="clip-flant5: replay the step from a CUDA graph (ClipT5Engine.score_tensors_graphed); "
                     "meant for small --batch, where ~700 launches of host work are the floor")
     ap.add_argument("--ncu", action="store_true", help="profiling pass: 2 device steps only, no JSON (run under ncu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the scores of the last timed step as DIR/scores.npy "
+                    "(float32; inputs are seeded, so two builds can be compared output for output)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.ncu):
+        ap.error("--dump-outputs writes what the engine's timed steps computed: not available with --impl reference or --ncu")
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, **arrays):
+    """Write each array as out_dir/<name>.npy in float32. An output larger than DUMP_MAX_BYTES in all is replaced by the same fixed,
+    seeded sample of its elements (in index order) on every run, so that dumps of two builds stay comparable element for element."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().float().cpu().reshape(-1)
+        keep = DUMP_MAX_BYTES // 4 // len(arrays)
+        if a.numel() > keep:
+            a = a[torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
 
 
 def measured_peaks():
@@ -259,20 +283,20 @@ def _tf_version():
 
 def run_reference(args, rank, world):
     """`--impl reference`: the reference's CPU path on this box's host cores, on the engine arm's config (clip-flant5-xxl shapes), every
-    reported pair measured at full depth. A step = one (image, text) pair at batch 1 -- the bounded sample of the 64-pair batch that the CPU
-    finishes in seconds; `steps` is the number of pairs actually timed (the requested --steps is echoed as steps_requested) so that
-    ms_per_step x steps is the real timed region. BASELINE config 1 (xl, the reference's PNGs) is measured in the same run (`config1`)."""
+    reported pair measured at full depth. A step = one (image, text) pair at batch 1 -- a sample of the 64-pair batch that the CPU
+    finishes in seconds; --steps pairs are timed, so that ms_per_step x steps is the real timed region (the requested --steps is also
+    echoed as steps_requested). BASELINE config 1 (xl, the reference's PNGs) is measured in the same run (`config1`)."""
     if rank != 0:
         return
     t0 = time.perf_counter()
     if args.model.startswith("qwen"):
-        best = cpu_reference_qwen(args.model, timed_pairs=max(3, min(args.steps, 6)), budget_s=150.0, video=args.video, video_size=args.video_size)
+        best = cpu_reference_qwen(args.model, timed_pairs=args.steps, budget_s=float("inf"), video=args.video, video_size=args.video_size)
         metric = "VQAScore (video,text) pairs/sec @ qwen2.5-vl-7b, 16x224px" if args.video else "VQAScore (image,text) pairs/sec @ qwen2.5-vl-7b, 448px"
         workload = f"{args.model} VQAScore on the host CPU, one sample per generate() call"
         cfg1 = None
     else:
         cfg1 = cpu_reference_clipt5("clip-flant5-xl", args.text_len, 16, 0.0, config1=True)
-        best = cfg1 if args.config1 else cpu_reference_clipt5(args.model, args.text_len, timed_pairs=max(3, min(args.steps, 8)), budget_s=150.0)
+        best = cfg1 if args.config1 else cpu_reference_clipt5(args.model, args.text_len, timed_pairs=args.steps, budget_s=float("inf"))
         metric = "VQAScore (image,text) pairs/sec @ clip-flant5-xxl, 512px"
         workload = (f"{'clip-flant5-xl' if args.config1 else args.model} VQAScore: the engine arm's pairs (336px CLIP input, {args.text_len} ids incl. image slot, "
                     f"S_enc=672, labels [Yes,</s>]) one pair per step at batch 1 on the host CPU")
@@ -396,7 +420,7 @@ def run_job(args, rank, world, dev, cfg, eng):
     if rank == 0:
         sampler.start()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    steps = max(1, min(args.steps, 2))
+    steps = args.steps
     sync_all()
     ev0.record()
     for _ in range(steps):
@@ -409,6 +433,8 @@ def run_job(args, rank, world, dev, cfg, eng):
     ms_job = float(t) / steps
     clocks = sampler.stop() if rank == 0 else None
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, scores=out)
         assert out.numel() == N and bool(torch.isfinite(out).all()) and float(out.min()) >= 0 and float(out.max()) <= 1
         emit(dict(
             metric="VQAScore (image,text) pairs/sec @ clip-flant5-xxl, 512px", value=N / (ms_job * 1e-3), unit="pairs/s", n_gpus=world,
@@ -496,6 +522,8 @@ def run_engine(args, rank, local_rank, world):
     sync_all()
     ms_local = ev0.elapsed_time(ev1)
     launches = eng.last_launch_count()
+    if args.dump_outputs and rank == 0:          # now: with --graph, `out` is the graph's output buffer and the passes below overwrite it
+        dump_outputs(args.dump_outputs, scores=out)
     t = torch.tensor([ms_local], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -666,6 +694,8 @@ def run_engine_qwen(args, rank, local_rank, world):
     ev1.record()
     sync_all()
     launches = eng.last_launch_count()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scores=out)
     t = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

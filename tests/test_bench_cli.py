@@ -5,6 +5,10 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+import torch
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -30,7 +34,7 @@ def test_reference_arm_measures_every_reported_pair():
     ms_per_step x steps, the config-1 sub-object over the reference's 4 PNGs x 4 prompts, cores = what the process may really use."""
     line = _run_reference([])
     assert line["impl"] == "reference" and line["unit"] == "pairs/s" and line["value"] > 0 and line["gpu_launches"] == 0
-    assert line["steps"] == line["timing"]["pairs_timed"] >= 3 and line["steps_requested"] == 3
+    assert line["steps"] == line["timing"]["pairs_timed"] == 3 and line["steps_requested"] == 3
     assert abs(line["ms_per_step"] * line["steps"] / 1000.0 * line["value"] - line["steps"]) < 1e-6 * line["steps"] + 1e-9
     assert "MEASURED" in line["cpu_baseline"]["sample"] and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["value"] == line["value"] and line["e2e"]["h2d_bytes_per_step"] == 0
@@ -41,6 +45,7 @@ def test_reference_arm_measures_every_reported_pair():
 def test_reference_arm_qwen_follows_the_reference_loop():
     line = _run_reference(["--model", "qwen2.5-vl-7b"])
     assert line["impl"] == "reference" and line["value"] > 0 and "generate(max_new_tokens=1" in line["cpu_baseline"]["sample"]
+    assert line["steps"] == line["timing"]["pairs_timed"] == 3
 
 
 def test_reference_arm_qwen_video_shapes():
@@ -61,3 +66,45 @@ def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     out = subprocess.run([sys.executable, "bench.py", "--impl", "reference", "--gpus", "2"], capture_output=True, text=True, cwd=ROOT,
                          timeout=300, env=env)
     assert out.returncode == 0 and out.stdout == ""
+
+
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"], ["--ncu", "--dump-outputs", "d"]])
+def test_arguments_without_a_timed_engine_step_are_refused(extra, tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, cwd=tmp_path, timeout=120)
+    assert out.returncode == 2 and out.stdout == "" and not os.listdir(tmp_path), out.stderr[-2000:]
+
+
+def test_dump_outputs_writes_float32_and_a_fixed_sample_of_large_outputs(tmp_path, monkeypatch):
+    import bench
+    small, large = torch.linspace(0, 1, 7, dtype=torch.float64), torch.arange(1000, dtype=torch.float32)
+    bench.dump_outputs(str(tmp_path / "a"), scores=small)
+    got = np.load(tmp_path / "a" / "scores.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, small.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 400)                     # room for 100 float32 values
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), scores=large)
+    b, c = np.load(tmp_path / "b" / "scores.npy"), np.load(tmp_path / "c" / "scores.npy")
+    assert b.dtype == np.float32 and b.nbytes <= 400 and len(b) == 100 and np.array_equal(b, c)
+    assert np.all(np.diff(b) > 0) and set(b.tolist()) <= set(large.tolist())      # distinct elements, in index order
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_and_steps_are_the_timed_steps(tmp_path):
+    """Two runs with the same arguments see the same seeded inputs: the dumped scores of the last timed step agree, and the JSON line
+    reports exactly the requested number of timed steps."""
+    if not torch.cuda.is_available():
+        pytest.skip("no GPU")
+    lines, dumps = [], []
+    for steps in (1, 2):
+        d = tmp_path / f"run{steps}"
+        out = subprocess.run([sys.executable, "bench.py", "--model", "clip-flant5-xl", "--batch", "8", "--steps", str(steps), "--warmup", "1",
+                              "--no-hf-baseline", "--no-cpu-baseline", "--dump-outputs", str(d)], capture_output=True, text=True, cwd=ROOT,
+                             timeout=900)
+        assert out.returncode == 0, out.stderr[-2000:]
+        lines.append(json.loads(out.stdout))
+        dumps.append(np.load(d / "scores.npy"))
+    assert [ln["steps"] for ln in lines] == [1, 2]
+    for ln, s in zip(lines, dumps):
+        assert s.dtype == np.float32 and s.shape == (8,) and np.all(np.isfinite(s)) and np.all((s >= 0) & (s <= 1))
+        assert np.allclose(s[:4], ln["sample_scores"], atol=1e-6)
+    assert np.allclose(dumps[0], dumps[1], atol=1e-5), (dumps[0], dumps[1])
