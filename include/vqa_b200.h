@@ -270,6 +270,31 @@ int vqa_qwen_preprocess(const void* src, const int64_t* offsets, const int32_t* 
  * arguments). Either output pointer may be NULL. */
 int32_t vqa_resample_table(int32_t in_size, int32_t out_size, int32_t first, int32_t count, int32_t* bounds, int32_t* kk);
 
+/* Qwen2.5-VL video pre-processing on the device: for each video, smart_resize with its own pixel bounds, resize of every frame, /255,
+ * normalise, consecutive frames paired into temporal patches (a count that is not a multiple of temporal_patch repeats the last frame)
+ * and 14x14 patch rows in 2x2 merge-block order -- what Qwen2VLVideoProcessor(do_resize=False) does to qwen_vl_utils' frames.
+ *   src        DEVICE, video v = frames[v] packed HWC uint8 RGB frames of heights[v] x widths[v], back to back from byte offsets[v]
+ *   policy[v]  VQA_RESAMPLE_PIL (frames handed over as images: Pillow's bicubic, bit-exact) or VQA_RESAMPLE_TORCHVISION (decoded video
+ *              files: torchvision's antialiased bicubic on uint8 tensors, fp32 taps and intermediate, clamp + round-half-even)
+ *   min_pixels / max_pixels  HOST [n_videos], the smart_resize bounds of each video
+ *   grid_thw   HOST [n_videos][3] (plan only) = (ceil(frames / temporal_patch), h / patch, w / patch)
+ *   out        DEVICE [total_patches, 3*temporal_patch*patch^2], video v's rows after those of videos 0..v-1
+ * vqa_qwen_video_preprocess_plan is host-only. At most 65535 frames per call. workspace / host_staging as for vqa_clip_preprocess. */
+#define VQA_RESAMPLE_PIL 0
+#define VQA_RESAMPLE_TORCHVISION 1
+int vqa_qwen_video_preprocess_plan(const int32_t* heights, const int32_t* widths, const int32_t* frames, const int32_t* policy,
+                                   int32_t n_videos, int32_t patch, int32_t temporal_patch, int32_t merge, const int64_t* min_pixels,
+                                   const int64_t* max_pixels, int32_t* grid_thw, int64_t* total_patches, size_t* workspace_bytes);
+int vqa_qwen_video_preprocess(const void* src, const int64_t* offsets, const int32_t* heights, const int32_t* widths, const int32_t* frames,
+                              const int32_t* policy, int32_t n_videos, int32_t patch, int32_t temporal_patch, int32_t merge,
+                              const int64_t* min_pixels, const int64_t* max_pixels, const float* mean, const float* stdv, void* out,
+                              int32_t out_dtype, void* workspace, size_t workspace_bytes, void* host_staging, void* stream);
+
+/* Host-only helper: the fp32 tap table of one axis of the VQA_RESAMPLE_TORCHVISION resize, exactly as vqa_qwen_video_preprocess builds
+ * it. bounds [count][2] = (first source index, taps used); taps [count][ksize]; *fma = 1 when the pass over this axis accumulates
+ * acc = fma(px, tap, acc), 0 when it computes acc + round(px * tap); returns ksize (0 = bad arguments). Pointers may be NULL. */
+int32_t vqa_resample_table_tv(int32_t in_size, int32_t out_size, int32_t first, int32_t count, int32_t* bounds, float* taps, int32_t* fma);
+
 /* ---- kernel-level entry points (used by tests/ and bench.py to exercise single kernels through the same ABI) ---- */
 
 /* C[M,N] = epilogue(A[M,K] . W[N,K]^T); all DEVICE bf16 row-major. epilogue: 0 store, 1 quick_gelu, 2 gelu(erf),

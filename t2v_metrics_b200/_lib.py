@@ -21,9 +21,11 @@ ABI_SYMBOLS = [
     "vqa_qwen_preprocess", "vqa_clipt5_debug_layout", "vqa_qwen25vl_debug_layout", "vqa_set_gemm_schedule",
     "vqa_qwen25vl_topk", "vqa_op_gemm_bf16_normfuse",
     "vqa_qwen25vl_packed_workspace_bytes", "vqa_qwen25vl_score_packed", "vqa_debug_max_active_clusters", "vqa_op_attention_d128_ex", "vqa_op_gemm_bf16_grouped", "vqa_op_gemm_bf16_splitk",
+    "vqa_qwen_video_preprocess_plan", "vqa_qwen_video_preprocess", "vqa_resample_table_tv",
 ]
 
 VQA_DTYPE_BF16, VQA_DTYPE_F32, VQA_DTYPE_I32 = 0, 1, 2
+VQA_RESAMPLE_PIL, VQA_RESAMPLE_TORCHVISION = 0, 1
 
 
 class VqaClipT5Config(C.Structure):
@@ -147,6 +149,15 @@ def load() -> C.CDLL:
     lib.vqa_debug_max_active_clusters.restype = C.c_int
     lib.vqa_resample_table.argtypes = [i32, i32, i32, i32, C.POINTER(i32), C.POINTER(i32)]
     lib.vqa_resample_table.restype = i32
+    lib.vqa_qwen_video_preprocess_plan.argtypes = [C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), i32, i32, i32, i32,
+                                                   C.POINTER(i64), C.POINTER(i64), C.POINTER(i32), C.POINTER(i64), C.POINTER(C.c_size_t)]
+    lib.vqa_qwen_video_preprocess_plan.restype = C.c_int
+    lib.vqa_qwen_video_preprocess.argtypes = [vp, C.POINTER(i64), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), C.POINTER(i32), i32, i32,
+                                              i32, i32, C.POINTER(i64), C.POINTER(i64), C.POINTER(C.c_float), C.POINTER(C.c_float), vp, i32,
+                                              vp, C.c_size_t, vp, vp]
+    lib.vqa_qwen_video_preprocess.restype = C.c_int
+    lib.vqa_resample_table_tv.argtypes = [i32, i32, i32, i32, C.POINTER(i32), C.POINTER(C.c_float), C.POINTER(i32)]
+    lib.vqa_resample_table_tv.restype = i32
     _lib = lib
     return lib
 

@@ -43,9 +43,13 @@ struct PreImage {            // one per image, lives in the workspace (device) a
     long long out_off;       // element offset of this image's output inside `out`
     int x_lo4, span4;        // groups of 4 canvas columns [x_lo4, x_lo4 + span4) the horizontal tap words touch
     int chunk_groups;        // groups of 4 canvas rows staged per pass (1 or 2)
+    int policy;              // PRE_PIL (22-bit fixed point, uint8 intermediate) or PRE_TORCHVISION (fp32 taps and intermediate)
+    int hfma, vfma;          // PRE_TORCHVISION: the pass accumulates with fma (1) or with a rounded product then an add (0)
+    int t_lo, t_hi;          // PRE_QWEN_PATCHES: the temporal slots [t_lo, t_hi) this frame is written to
 };
 
 enum PreLayout { PRE_CHW = 0, PRE_QWEN_PATCHES = 1 };
+enum PrePolicy { PRE_PIL = 0, PRE_TORCHVISION = 1 };
 struct PrePatchGeom { int patch, merge, temporal; };     // PRE_QWEN_PATCHES only
 
 // ---------------------------------------------------------------------------------------------- host: Pillow's coefficient tables
@@ -131,6 +135,84 @@ inline int pre_pack_table(const int* bounds, const int* kk, int count, int ksize
     return np;
 }
 
+// ---------------------------------------------------------------------------------------------- host: torch's antialiased bicubic taps
+// What torchvision.transforms.functional.resize(uint8 tensor, BICUBIC, antialias=True) computes: a cast to fp32, then
+// F.interpolate(mode="bicubic", antialias=True) (aten/src/ATen/native/cpu/UpSampleKernel.cpp, HelperInterpCubic with a = -0.5 and
+// _compute_indices_min_size_weights_aa), then clamp(0, 255) and round-half-even back to uint8. The taps below reproduce torch's CPU
+// build (x86-64, compiled with FMA contraction) bit for bit: the filter polynomials as fused multiply-adds, `center -/+ support` in
+// fp32 before the + 0.5 in double, the argument (x - center) in fp32 then (+ 0.5) * invscale in double, weights normalised by their
+// fp32 sum. The passes run width first, then height, each over an fp32 intermediate. torch accumulates `acc += px * w` sequentially
+// from the first tap; its build contracts that to an fma on upscaled axes and keeps a rounded product on downscaled ones (probed on
+// torch 2.11 CPU), which is what `fma` returns. Both are a compiler's choice, not part of torch's API: a build that contracts
+// differently moves results by one grey level where the fp32 sum sits at a rounding tie (measured in the tests).
+inline float pre_tv_cubic(float x) {
+    const float a = -0.5f;
+    x = std::fabs(x);
+    if (x < 1.0f) return std::fmaf(std::fmaf(a + 2.0f, x, -(a + 3.0f)) * x, x, 1.0f);
+    if (x < 2.0f) return std::fmaf(std::fmaf(std::fmaf(a, x, -5.0f * a), x, 8.0f * a), x, -4.0f * a);
+    return 0.0f;
+}
+
+// Taps of output pixels [first, first + count) of an in_size -> out_size resize. Appends (xmin, n) bounds then count * ksize taps (fp32
+// bit patterns) to `tab`; returns ksize. `fma`: whether the passes over this axis accumulate with fma.
+inline int pre_build_table_tv(int in_size, int out_size, int first, int count, std::vector<int>& tab, int* fma) {
+    const float scale = (float)in_size / (float)out_size;
+    const float support = scale >= 1.0f ? 2.0f * scale : 2.0f;           // (interp_size * 0.5) * scale, interp_size = 4
+    const float invscale = scale >= 1.0f ? 1.0f / scale : 1.0f;
+    const int ksize = (int)std::ceil(support) * 2 + 1;
+    const size_t base = tab.size();
+    tab.resize(base + (size_t)count * 2 + (size_t)count * ksize, 0);
+    int* bounds = tab.data() + base;
+    float* kk = reinterpret_cast<float*>(bounds + (size_t)count * 2);
+    for (int i = 0; i < count; ++i) {
+        const int xx = first + i;
+        const float center = (float)((double)scale * (xx + 0.5));
+        int xmin = (int)((double)(center - support) + 0.5);
+        if (xmin < 0) xmin = 0;
+        int xmax = (int)((double)(center + support) + 0.5);
+        if (xmax > in_size) xmax = in_size;
+        int n = xmax - xmin;
+        if (n > ksize) n = ksize;
+        if (n < 0) n = 0;
+        float* w = kk + (size_t)i * ksize;
+        float total = 0.0f;
+        for (int j = 0; j < n; ++j) {
+            const float d = (float)(j + xmin) - center;
+            w[j] = pre_tv_cubic((float)(((double)d + 0.5) * (double)invscale));
+            total += w[j];
+        }
+        if (total != 0.0f)
+            for (int j = 0; j < n; ++j) w[j] /= total;
+        bounds[2 * i] = xmin;
+        bounds[2 * i + 1] = n;
+    }
+    if (fma) *fma = out_size > in_size ? 1 : 0;
+    return ksize;
+}
+
+// pre_pack_table for fp32 taps: start4[count], last4[count], then taps[count][np][4] (fp32, aligned to the same groups of four source
+// pixels, zero where the window has no tap: a zero tap adds an exact zero under either accumulation). Returns np.
+inline int pre_pack_table_tv(const int* bounds, const float* kk, int count, int ksize, std::vector<int>& tab) {
+    int np = 1;
+    for (int i = 0; i < count; ++i) {
+        const int x0 = bounds[2 * i], n = bounds[2 * i + 1];
+        const int words = n > 0 ? (x0 + n - 1) / 4 - x0 / 4 + 1 : 1;
+        if (words > np) np = words;
+    }
+    const size_t base = tab.size();
+    tab.resize(base + (size_t)count * 2 + (size_t)count * np * 4, 0);
+    int* start4 = tab.data() + base;
+    int* last4 = start4 + count;
+    float* taps = reinterpret_cast<float*>(last4 + count);
+    for (int i = 0; i < count; ++i) {
+        const int x0 = bounds[2 * i], n = bounds[2 * i + 1];
+        start4[i] = x0 / 4;
+        last4[i] = n > 0 ? (x0 + n - 1) / 4 : x0 / 4;
+        for (int x = 0; x < n; ++x) taps[((size_t)i * np) * 4 + (x0 + x) - 4 * start4[i]] = kk[(size_t)i * ksize + x];
+    }
+    return np;
+}
+
 // ---------------------------------------------------------------------------------------------- device
 __device__ __forceinline__ int pre_clip8(int v) {     // Resample.c clip8: table lookup of (v >> PRECISION_BITS) clamped to [0, 255]
     v >>= PRE_PRECISION_BITS;
@@ -154,9 +236,12 @@ __device__ __forceinline__ unsigned pre_finish(unsigned a0, unsigned a1, int a2)
 
 // LAYOUT PRE_CHW: out[c][y][x] per image ([3, out_h, out_w]). PRE_QWEN_PATCHES: the Qwen2-VL processor's patch rows
 // (image_processing_qwen2_vl.py:191-220): row ((by * gw/m + bx) * m + iy) * m + ix for the 14x14 patch at grid (by*m+iy, bx*m+ix),
-// column (c * temporal + t) * ps*ps + py * ps + px, the still frame written to every temporal slot t.
+// column (c * temporal + t) * ps*ps + py * ps + px, the frame written to temporal slots [t_lo, t_hi) (a still image: all of them).
+// Per image, `policy` selects the resample: PRE_PIL (the dp4a fixed-point passes above, uint8 intermediate) or PRE_TORCHVISION (fp32
+// taps, fp32 intermediate, clamp + round-half-even at the end; see pre_build_table_tv). Both share the staging, the band and the
+// output stage; only the two filter passes differ.
 template <typename OUT, int LAYOUT>
-__global__ void __launch_bounds__(PRE_THREADS)
+__global__ void __launch_bounds__(PRE_THREADS, 3)     // 3 CTAs an SM, as before the fp32 passes joined: no spills at 79 registers
 image_preprocess_kernel(const uint8_t* __restrict__ src, const PreImage* __restrict__ images, const int* __restrict__ tables,
                         uchar3 background, float3 mean, float3 stdv, PrePatchGeom geom, OUT* __restrict__ out) {
     pdl_launch_dependents();
@@ -168,8 +253,10 @@ image_preprocess_kernel(const uint8_t* __restrict__ src, const PreImage* __restr
     const int ny = min(im.tile_rows, im.out_h - y0);
     const int chunk_rows = im.chunk_groups * 4;
     float* lut = reinterpret_cast<float*>(pre_smem);                          // [3][256] normalised value of every grey level
+    const bool tv = im.policy == PRE_TORCHVISION;
     uint32_t* band = pre_smem + 768;                                           // [3][band_groups][out_w]: 4 canvas rows per word
-    uint32_t* stage = band + (size_t)3 * im.band_groups * out_w;               // [3][chunk_rows][span4]: 4 canvas columns per word
+    float* bandf = reinterpret_cast<float*>(band);                             // PRE_TORCHVISION: [3][band_groups * 4][out_w] fp32
+    uint32_t* stage = band + (size_t)3 * im.band_groups * out_w * (tv ? 4 : 1);  // [3][chunk_rows][span4]: 4 canvas columns per word
     const int* hstart = tables + im.htab;
     const uint32_t* hwords = reinterpret_cast<const uint32_t*>(hstart + 2 * out_w);
     const int* vstart = tables + im.vtab;
@@ -230,8 +317,41 @@ image_preprocess_kernel(const uint8_t* __restrict__ src, const PreImage* __restr
             }
         }
         __syncthreads();
+        // ---- horizontal pass, torchvision policy: fp32 taps over the staged bytes, sequential from the window's first tap
+        if (tv && grp < ngc) {
+            const float* htaps = reinterpret_cast<const float*>(hstart + 2 * out_w);
+            for (int xx = lane_x; xx < out_w; xx += PRE_XL) {
+                const int s4 = hstart[xx] - im.x_lo4;
+                const float* kw = htaps + (size_t)xx * im.hnp * 4;
+                float acc[4][3];
+#pragma unroll
+                for (int q = 0; q < 4; ++q)
+#pragma unroll
+                    for (int c = 0; c < 3; ++c) acc[q][c] = 0.0f;
+                for (int pw = 0; pw < im.hnp; ++pw) {
+                    float k[4];
+#pragma unroll
+                    for (int b = 0; b < 4; ++b) k[b] = __ldg(kw + pw * 4 + b);
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+#pragma unroll
+                        for (int c = 0; c < 3; ++c) {
+                            const uint32_t px = stage[(size_t)(c * chunk_rows + grp * 4 + q) * im.span4 + s4 + pw];
+#pragma unroll
+                            for (int b = 0; b < 4; ++b) {
+                                const float p = (float)((px >> (8 * b)) & 0xffu);
+                                acc[q][c] = im.hfma ? __fmaf_rn(p, k[b], acc[q][c]) : __fadd_rn(acc[q][c], __fmul_rn(p, k[b]));
+                            }
+                        }
+                }
+#pragma unroll
+                for (int c = 0; c < 3; ++c)
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) bandf[((size_t)c * im.band_groups * 4 + (cg + grp) * 4 + q) * out_w + xx] = acc[q][c];
+            }
+        }
         // ---- horizontal pass (ImagingResampleHorizontal_8bpc): thread = one output column x one group of 4 canvas rows
-        if (grp < ngc) {
+        if (!tv && grp < ngc) {
             for (int xx = lane_x; xx < out_w; xx += PRE_XL) {
                 const int s4 = hstart[xx] - im.x_lo4;
                 const uint32_t* kw = hwords + (size_t)xx * im.hnp * 3;
@@ -273,22 +393,41 @@ image_preprocess_kernel(const uint8_t* __restrict__ src, const PreImage* __restr
         const int y = y0 + yy;
         const int gs = vstart[y] - g0;
         const uint32_t* kw = vwords + (size_t)y * im.vnp * 3;
+        const float* kf = reinterpret_cast<const float*>(vwords) + (size_t)y * im.vnp * 4;
+        const int vn = vlast[y] - vstart[y] + 1;            // torchvision policy: only groups this CTA staged (fp32 garbage is not inert)
         for (int xx = lane_x; xx < out_w; xx += PRE_XL) {
-            unsigned a0[3] = {0, 0, 0}, a1[3] = {0, 0, 0};
-            int a2[3] = {0, 0, 0};
-            for (int pw = 0; pw < im.vnp; ++pw) {
-                const uint32_t d0 = __ldg(kw + pw * 3), d1 = __ldg(kw + pw * 3 + 1), d2 = __ldg(kw + pw * 3 + 2);
-#pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    const uint32_t px = band[((size_t)c * im.band_groups + gs + pw) * out_w + xx];
-                    a0[c] = pre_dp4a_uu(px, d0, a0[c]);
-                    a1[c] = pre_dp4a_uu(px, d1, a1[c]);
-                    a2[c] = pre_dp4a_us(px, d2, a2[c]);
-                }
-            }
             float v[3];
+            if (tv) {
+                float acc[3] = {0.0f, 0.0f, 0.0f};
+                for (int pw = 0; pw < vn; ++pw) {
 #pragma unroll
-            for (int c = 0; c < 3; ++c) v[c] = lut[c * 256 + pre_finish(a0[c], a1[c], a2[c])];
+                    for (int b = 0; b < 4; ++b) {
+                        const float k = __ldg(kf + pw * 4 + b);
+#pragma unroll
+                        for (int c = 0; c < 3; ++c) {
+                            const float p = bandf[((size_t)c * im.band_groups * 4 + (gs + pw) * 4 + b) * out_w + xx];
+                            acc[c] = im.vfma ? __fmaf_rn(p, k, acc[c]) : __fadd_rn(acc[c], __fmul_rn(p, k));
+                        }
+                    }
+                }
+#pragma unroll
+                for (int c = 0; c < 3; ++c) v[c] = lut[c * 256 + (int)rintf(fminf(fmaxf(acc[c], 0.0f), 255.0f))];
+            } else {
+                unsigned a0[3] = {0, 0, 0}, a1[3] = {0, 0, 0};
+                int a2[3] = {0, 0, 0};
+                for (int pw = 0; pw < im.vnp; ++pw) {
+                    const uint32_t d0 = __ldg(kw + pw * 3), d1 = __ldg(kw + pw * 3 + 1), d2 = __ldg(kw + pw * 3 + 2);
+#pragma unroll
+                    for (int c = 0; c < 3; ++c) {
+                        const uint32_t px = band[((size_t)c * im.band_groups + gs + pw) * out_w + xx];
+                        a0[c] = pre_dp4a_uu(px, d0, a0[c]);
+                        a1[c] = pre_dp4a_uu(px, d1, a1[c]);
+                        a2[c] = pre_dp4a_us(px, d2, a2[c]);
+                    }
+                }
+#pragma unroll
+                for (int c = 0; c < 3; ++c) v[c] = lut[c * 256 + pre_finish(a0[c], a1[c], a2[c])];
+            }
             if constexpr (LAYOUT == PRE_CHW) {
 #pragma unroll
                 for (int c = 0; c < 3; ++c) {
@@ -302,7 +441,7 @@ image_preprocess_kernel(const uint8_t* __restrict__ src, const PreImage* __restr
                 OUT* q = dst + row * (size_t)(3 * geom.temporal * pp) + py * ps + px_;
 #pragma unroll
                 for (int c = 0; c < 3; ++c)
-                    for (int t = 0; t < geom.temporal; ++t) {
+                    for (int t = im.t_lo; t < im.t_hi; ++t) {
                         if constexpr (sizeof(OUT) == 4) q[(size_t)(c * geom.temporal + t) * pp] = v[c];
                         else q[(size_t)(c * geom.temporal + t) * pp] = __float2bfloat16_rn(v[c]);
                     }
@@ -322,26 +461,34 @@ struct PrePlan {
     size_t bytes() const { return images_bytes() + tables.size() * sizeof(int); }
 };
 
-struct PreTableKey { int ch, cw, nh, nw, top, left, oh, ow, htab, vtab, hnp, vnp, tile, band_groups, x_lo4, span4, chunk_groups; };
-inline size_t pre_smem_bytes(int band_groups, int out_w, int chunk_groups, int span4) {
-    return 768 * sizeof(float) + ((size_t)3 * band_groups * out_w + (size_t)3 * chunk_groups * 4 * span4) * sizeof(uint32_t);
+struct PreTableKey {
+    int ch, cw, nh, nw, top, left, oh, ow, htab, vtab, hnp, vnp, tile, band_groups, x_lo4, span4, chunk_groups, policy, hfma, vfma;
+};
+inline size_t pre_smem_bytes(int band_groups, int out_w, int chunk_groups, int span4, int policy = PRE_PIL) {
+    const size_t band_words = (size_t)3 * band_groups * out_w * (policy == PRE_TORCHVISION ? 4 : 1);   // fp32 rows vs 4 uint8 rows a word
+    return 768 * sizeof(float) + (band_words + (size_t)3 * chunk_groups * 4 * span4) * sizeof(uint32_t);
 }
 
 // Tables + band geometry for "resize the ch x cw canvas to nh x nw, keep the oh x ow window at (top, left)"; shared between images
 // with the same geometry. Returns nullptr (plan.error set) when the filter windows cannot fit the shared-memory budget.
 inline const PreTableKey* pre_tables(PrePlan& plan, std::vector<PreTableKey>& cache, int ch, int cw, int nh, int nw, int top, int left,
-                                     int oh, int ow) {
+                                     int oh, int ow, int policy = PRE_PIL) {
     for (const PreTableKey& k : cache)
-        if (k.ch == ch && k.cw == cw && k.nh == nh && k.nw == nw && k.top == top && k.left == left && k.oh == oh && k.ow == ow) return &k;
-    PreTableKey k{ch, cw, nh, nw, top, left, oh, ow, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+        if (k.ch == ch && k.cw == cw && k.nh == nh && k.nw == nw && k.top == top && k.left == left && k.oh == oh && k.ow == ow &&
+            k.policy == policy)
+            return &k;
+    PreTableKey k{ch, cw, nh, nw, top, left, oh, ow, 0, 0, 0, 0, 0, 0, 0, 0, 0, policy, 0, 0};
     std::vector<int> raw;
-    int ks = pre_build_table(cw, nw, left, ow, raw);
+    const bool tv = policy == PRE_TORCHVISION;
+    int ks = tv ? pre_build_table_tv(cw, nw, left, ow, raw, &k.hfma) : pre_build_table(cw, nw, left, ow, raw);
     k.htab = (int)plan.tables.size();
-    k.hnp = pre_pack_table(raw.data(), raw.data() + (size_t)ow * 2, ow, ks, plan.tables);
+    k.hnp = tv ? pre_pack_table_tv(raw.data(), reinterpret_cast<const float*>(raw.data() + (size_t)ow * 2), ow, ks, plan.tables)
+               : pre_pack_table(raw.data(), raw.data() + (size_t)ow * 2, ow, ks, plan.tables);
     raw.clear();
-    ks = pre_build_table(ch, nh, top, oh, raw);
+    ks = tv ? pre_build_table_tv(ch, nh, top, oh, raw, &k.vfma) : pre_build_table(ch, nh, top, oh, raw);
     k.vtab = (int)plan.tables.size();
-    k.vnp = pre_pack_table(raw.data(), raw.data() + (size_t)oh * 2, oh, ks, plan.tables);
+    k.vnp = tv ? pre_pack_table_tv(raw.data(), reinterpret_cast<const float*>(raw.data() + (size_t)oh * 2), oh, ks, plan.tables)
+               : pre_pack_table(raw.data(), raw.data() + (size_t)oh * 2, oh, ks, plan.tables);
     const int* hstart = plan.tables.data() + k.htab;
     const int* vstart = plan.tables.data() + k.vtab;
     k.x_lo4 = hstart[0];                           // windows are monotonic: first word of the first output .. last word of the last
@@ -355,8 +502,8 @@ inline const PreTableKey* pre_tables(PrePlan& plan, std::vector<PreTableKey>& ca
             const int groups = vstart[y1] + k.vnp - vstart[y0];
             if (groups > band) band = groups;
         }
-        for (chunk = PRE_RG; chunk > 1 && pre_smem_bytes(band, ow, chunk, k.span4) > (size_t)PRE_MAX_SMEM; chunk >>= 1) {}
-        if (pre_smem_bytes(band, ow, chunk, k.span4) <= (size_t)PRE_MAX_SMEM) break;
+        for (chunk = PRE_RG; chunk > 1 && pre_smem_bytes(band, ow, chunk, k.span4, policy) > (size_t)PRE_MAX_SMEM; chunk >>= 1) {}
+        if (pre_smem_bytes(band, ow, chunk, k.span4, policy) <= (size_t)PRE_MAX_SMEM) break;
     }
     if (tile < 1) { plan.error = "image too large for the device resize (filter windows exceed shared memory)"; return nullptr; }
     k.tile = tile; k.band_groups = band; k.chunk_groups = chunk;
@@ -368,9 +515,10 @@ inline void pre_finish_image(PrePlan& plan, PreImage& im, const PreTableKey& k) 
     im.htab = k.htab; im.vtab = k.vtab; im.hnp = k.hnp; im.vnp = k.vnp;
     im.tile_rows = k.tile; im.band_groups = k.band_groups; im.out_h = k.oh; im.out_w = k.ow;
     im.x_lo4 = k.x_lo4; im.span4 = k.span4; im.chunk_groups = k.chunk_groups;
+    im.policy = k.policy; im.hfma = k.hfma; im.vfma = k.vfma;
     const int tiles = (k.oh + k.tile - 1) / k.tile;
     if (tiles > plan.max_tiles) plan.max_tiles = tiles;
-    const size_t sm = pre_smem_bytes(k.band_groups, k.ow, k.chunk_groups, k.span4);
+    const size_t sm = pre_smem_bytes(k.band_groups, k.ow, k.chunk_groups, k.span4, k.policy);
     if (sm > plan.smem) plan.smem = sm;
 }
 
@@ -445,8 +593,55 @@ inline bool pre_plan_qwen(const int32_t* heights, const int32_t* widths, const i
         if (!k) return false;
         pre_finish_image(plan, im, *k);
         im.out_off = rows * row_elems;
+        im.t_lo = 0; im.t_hi = temporal;
         if (grid_hw) { grid_hw[2 * i] = rh / patch; grid_hw[2 * i + 1] = rw / patch; }
         rows += (long long)(rh / patch) * (rw / patch);
+    }
+    if (total_rows) *total_rows = rows;
+    return true;
+}
+
+// Qwen videos: video v is frames[v] uint8 HWC frames of heights[v] x widths[v], stored back to back from offsets[v]. smart_resize with
+// the video's own pixel bounds, resample policy policy[v] (PRE_PIL: frames given as images, each resized by PIL; PRE_TORCHVISION:
+// decoded files, resized by torchvision), then consecutive frames form one temporal patch: frame f goes to temporal slot f % temporal
+// of grid step f / temporal. A count that is not a multiple of `temporal` is completed by repeating the last frame, which is done by
+// writing that frame to all the remaining slots of its step. One PreImage per frame; video v's rows start at sum_{u<v} t_u gh_u gw_u.
+// grid_thw[v] = (t, gh, gw).
+inline bool pre_plan_qwen_video(const int32_t* heights, const int32_t* widths, const int32_t* frames, const int32_t* policy,
+                                const int64_t* offsets, int n, int patch, int merge, int temporal, const int64_t* min_pixels,
+                                const int64_t* max_pixels, PrePlan& plan, int32_t* grid_thw, long long* total_rows) {
+    std::vector<PreTableKey> cache;
+    cache.reserve(n);
+    long long rows = 0, entries = 0;
+    const long long row_elems = 3LL * temporal * patch * patch;
+    for (int v = 0; v < n; ++v) entries += frames[v] > 0 ? frames[v] : 0;
+    if (entries > 65535) { plan.error = "too many frames in one call (at most 65535)"; return false; }
+    plan.images.reserve((size_t)entries);
+    for (int v = 0; v < n; ++v) {
+        const int h = heights[v], w = widths[v], nf = frames[v];
+        if (h <= 0 || w <= 0 || nf <= 0) { plan.error = "video with non-positive size or no frames"; return false; }
+        if (policy[v] != PRE_PIL && policy[v] != PRE_TORCHVISION) { plan.error = "unknown resample policy"; return false; }
+        if (min_pixels[v] <= 0 || max_pixels[v] < min_pixels[v]) { plan.error = "bad pixel bounds"; return false; }
+        int rh, rw;
+        if (!pre_smart_resize(h, w, patch * merge, min_pixels[v], max_pixels[v], rh, rw)) {
+            plan.error = "absolute aspect ratio must be smaller than 200";
+            return false;
+        }
+        const PreTableKey* k = pre_tables(plan, cache, h, w, rh, rw, 0, 0, rh, rw, policy[v]);
+        if (!k) return false;
+        const int gh = rh / patch, gw = rw / patch, gt = (nf + temporal - 1) / temporal;
+        for (int f = 0; f < nf; ++f) {
+            PreImage im{};
+            im.src_off = offsets[v] + (long long)f * h * w * 3; im.h = h; im.w = w;
+            im.canvas_h = h; im.canvas_w = w;
+            pre_finish_image(plan, im, *k);
+            im.out_off = (rows + (long long)(f / temporal) * gh * gw) * row_elems;
+            im.t_lo = f % temporal;
+            im.t_hi = f == nf - 1 ? temporal : im.t_lo + 1;
+            plan.images.push_back(im);
+        }
+        if (grid_thw) { grid_thw[3 * v] = gt; grid_thw[3 * v + 1] = gh; grid_thw[3 * v + 2] = gw; }
+        rows += (long long)gt * gh * gw;
     }
     if (total_rows) *total_rows = rows;
     return true;

@@ -1429,3 +1429,58 @@ extern "C" int32_t vqa_resample_table(int32_t in_size, int32_t out_size, int32_t
     if (kk) memcpy(kk, tab.data() + (size_t)count * 2, (size_t)count * ksize * sizeof(int));
     return ksize;
 }
+
+// ---------------------------------------------------------------------------------------------- Qwen video pre-processing
+extern "C" int vqa_qwen_video_preprocess_plan(const int32_t* heights, const int32_t* widths, const int32_t* frames, const int32_t* policy,
+                                              int32_t n_videos, int32_t patch, int32_t temporal_patch, int32_t merge,
+                                              const int64_t* min_pixels, const int64_t* max_pixels, int32_t* grid_thw,
+                                              int64_t* total_patches, size_t* workspace_bytes) {
+    if (!heights || !widths || !frames || !policy || !min_pixels || !max_pixels || n_videos <= 0 || patch <= 0 || merge <= 0 ||
+        temporal_patch <= 0)
+        return fail(nullptr, VQA_ERR_INVALID_ARG, "bad argument");
+    PrePlan plan;
+    std::vector<int64_t> off(n_videos, 0);
+    long long rows = 0;
+    if (!pre_plan_qwen_video(heights, widths, frames, policy, off.data(), n_videos, patch, merge, temporal_patch, min_pixels, max_pixels,
+                             plan, grid_thw, &rows))
+        return fail(nullptr, VQA_ERR_INVALID_ARG, plan.error);
+    if (total_patches) *total_patches = rows;
+    if (workspace_bytes) *workspace_bytes = plan.bytes();
+    return VQA_OK;
+}
+
+extern "C" int vqa_qwen_video_preprocess(const void* src, const int64_t* offsets, const int32_t* heights, const int32_t* widths,
+                                         const int32_t* frames, const int32_t* policy, int32_t n_videos, int32_t patch,
+                                         int32_t temporal_patch, int32_t merge, const int64_t* min_pixels, const int64_t* max_pixels,
+                                         const float* mean, const float* stdv, void* out, int32_t out_dtype, void* workspace,
+                                         size_t workspace_bytes, void* host_staging, void* stream) {
+    if (!src || !offsets || !heights || !widths || !frames || !policy || !min_pixels || !max_pixels || !mean || !stdv || !out || !workspace)
+        return fail(nullptr, VQA_ERR_INVALID_ARG, "null pointer");
+    if (n_videos <= 0 || patch <= 0 || merge <= 0 || temporal_patch <= 0) return fail(nullptr, VQA_ERR_INVALID_ARG, "bad argument");
+    if (out_dtype != VQA_DTYPE_F32 && out_dtype != VQA_DTYPE_BF16) return fail(nullptr, VQA_ERR_INVALID_ARG, "out_dtype must be f32 or bf16");
+    PrePlan plan;
+    if (!pre_plan_qwen_video(heights, widths, frames, policy, offsets, n_videos, patch, merge, temporal_patch, min_pixels, max_pixels, plan,
+                             nullptr, nullptr))
+        return fail(nullptr, VQA_ERR_INVALID_ARG, plan.error);
+    const uint8_t no_bg[3] = {0, 0, 0};
+    return pre_launch<PRE_QWEN_PATCHES>(plan, src, (int)plan.images.size(), no_bg, mean, stdv, PrePatchGeom{patch, merge, temporal_patch}, out,
+                                        out_dtype, workspace, workspace_bytes, host_staging, reinterpret_cast<cudaStream_t>(stream));
+}
+
+// Host-only: the fp32 tap table of one axis of the torchvision-policy resize, exactly as vqa_qwen_video_preprocess builds it (for CPU
+// replays of the kernel's arithmetic). bounds: [count][2] (first source index, taps used), taps: [count][ksize] with ksize = return value
+// (call with taps = NULL to size it); *fma = 1 when the pass over this axis accumulates with fma, 0 when it rounds each product first.
+extern "C" int32_t vqa_resample_table_tv(int32_t in_size, int32_t out_size, int32_t first, int32_t count, int32_t* bounds, float* taps,
+                                         int32_t* fma) {
+    if (in_size <= 0 || out_size <= 0 || first < 0 || count <= 0 || first + count > out_size) {
+        fail(nullptr, VQA_ERR_INVALID_ARG, "bad resample table request");
+        return 0;
+    }
+    std::vector<int> tab;
+    int f = 0;
+    const int ksize = pre_build_table_tv(in_size, out_size, first, count, tab, &f);
+    if (bounds) memcpy(bounds, tab.data(), (size_t)count * 2 * sizeof(int));
+    if (taps) memcpy(taps, tab.data() + (size_t)count * 2, (size_t)count * ksize * sizeof(float));
+    if (fma) *fma = f;
+    return ksize;
+}

@@ -507,6 +507,90 @@ def qwen_preprocess_u8(images: Sequence[torch.Tensor], device, patch: int = 14, 
     return out, grids
 
 
+def _video_arrays(videos, policies, min_pixels, max_pixels):
+    n = len(videos)
+    assert n > 0 and len(policies) == n and len(min_pixels) == n and len(max_pixels) == n
+    fs, hs, ws, offs, total = [], [], [], [], 0
+    for v in videos:
+        assert v.dtype == torch.uint8 and v.dim() == 4 and v.shape[3] == 3, "videos must be uint8 [frames, h, w, 3]"
+        fs.append(int(v.shape[0])); hs.append(int(v.shape[1])); ws.append(int(v.shape[2])); offs.append(total)
+        total += int(v.numel())
+    i32 = lambda xs: (C.c_int32 * n)(*[int(x) for x in xs])
+    i64 = lambda xs: (C.c_int64 * n)(*[int(x) for x in xs])
+    return dict(F=i32(fs), H=i32(hs), W=i32(ws), P=i32(policies), MN=i64(min_pixels), MX=i64(max_pixels), O=i64(offs), total=total)
+
+
+def qwen_video_preprocess_plan(sizes_fhw: Sequence[Sequence[int]], policies: Sequence[int], min_pixels: Sequence[int],
+                               max_pixels: Sequence[int], patch: int = 14, temporal_patch: int = 2, merge: int = 2):
+    """Host-only geometry of the Qwen video pre-processing: (frames, h, w) per video -> ([(t, gh, gw), ...], total patch rows,
+    workspace bytes)."""
+    lib = _lib.load()
+    n = len(sizes_fhw)
+    a = _video_arrays([torch.empty(int(f), int(h), int(w), 3, dtype=torch.uint8, device="meta") for f, h, w in sizes_fhw], policies,
+                      min_pixels, max_pixels)
+    grid = (C.c_int32 * (3 * n))()
+    total, wsb = C.c_int64(0), C.c_size_t(0)
+    _check(lib.vqa_qwen_video_preprocess_plan(a["H"], a["W"], a["F"], a["P"], n, patch, temporal_patch, merge, a["MN"], a["MX"], grid,
+                                              C.byref(total), C.byref(wsb)), None, "vqa_qwen_video_preprocess_plan")
+    return [tuple(int(grid[3 * i + k]) for k in range(3)) for i in range(n)], int(total.value), int(wsb.value)
+
+
+def qwen_video_preprocess_u8(videos: Sequence[torch.Tensor], policies: Sequence[int], device, min_pixels: Sequence[int],
+                             max_pixels: Sequence[int], patch: int = 14, temporal_patch: int = 2, merge: int = 2, mean=CLIP_MEAN,
+                             std=CLIP_STD, out_dtype: torch.dtype = torch.float32):
+    """Sampled video frames (uint8 [frames, h, w, 3] RGB per video, host or device) -> (pixel_patches [sum t*gh*gw, 3*tp*patch^2] on
+    the device, [(t, gh, gw), ...]) by ONE kernel launch over every frame of every video: per-video smart_resize with its own pixel
+    bounds, the resample of `policies[v]` (_lib.VQA_RESAMPLE_PIL for frame stacks, _lib.VQA_RESAMPLE_TORCHVISION for decoded files),
+    /255, normalise, temporal pairing (an odd last frame fills both slots of its pair) and merge-order rows. Bit-identical to
+    qwen_utils.qwen_video_to_patches of pil_resize_frames / torchvision_resize_u8 (the latter up to fp32 ties, see
+    vqa_resample_table_tv)."""
+    lib = _lib.load()
+    dev = torch.device(device)
+    n = len(videos)
+    a = _video_arrays(videos, policies, min_pixels, max_pixels)
+    grid = (C.c_int32 * (3 * n))()
+    rows, need = C.c_int64(0), C.c_size_t(0)
+    _check(lib.vqa_qwen_video_preprocess_plan(a["H"], a["W"], a["F"], a["P"], n, patch, temporal_patch, merge, a["MN"], a["MX"], grid,
+                                              C.byref(rows), C.byref(need)), None, "vqa_qwen_video_preprocess_plan")
+    grids = [tuple(int(grid[3 * i + k]) for k in range(3)) for i in range(n)]
+    if all(v.is_cuda for v in videos):
+        src = videos[0].contiguous().view(-1) if n == 1 else torch.cat([v.contiguous().view(-1) for v in videos])
+    else:
+        stage = torch.empty(a["total"], dtype=torch.uint8, pin_memory=True)
+        o = 0
+        for v in videos:
+            stage[o:o + v.numel()] = v.contiguous().view(-1).cpu()
+            o += v.numel()
+        src = stage.to(dev, non_blocking=True)
+    out = torch.empty(int(rows.value), 3 * temporal_patch * patch * patch, dtype=out_dtype, device=dev)
+    wsb = torch.empty(max(int(need.value), 16), dtype=torch.uint8, device=dev)
+    ring = _staging(dev)
+    stage_buf = ring.acquire(wsb.numel())
+    with torch.cuda.device(dev):
+        rc = lib.vqa_qwen_video_preprocess(_ptr(src), a["O"], a["H"], a["W"], a["F"], a["P"], n, patch, temporal_patch, merge, a["MN"],
+                                           a["MX"], (C.c_float * 3)(*mean), (C.c_float * 3)(*std), _ptr(out),
+                                           _lib.VQA_DTYPE_F32 if out_dtype == torch.float32 else _lib.VQA_DTYPE_BF16, _ptr(wsb),
+                                           wsb.numel(), stage_buf.data_ptr(), _stream_ptr(dev))
+    ring.release(dev)
+    _check(rc, None, "vqa_qwen_video_preprocess")
+    return out, grids
+
+
+def resample_table_tv(in_size: int, out_size: int):
+    """Host-only: (bounds int32 [out, 2], taps fp32 [out, ksize], fma) of one axis of the torchvision-policy resize, as the kernel uses
+    them (vqa_resample_table_tv)."""
+    lib = _lib.load()
+    fma = C.c_int32(0)
+    ks = int(lib.vqa_resample_table_tv(in_size, out_size, 0, out_size, None, None, C.byref(fma)))
+    if ks == 0:
+        raise ValueError(_lib.last_error(None))
+    bounds = torch.zeros(out_size, 2, dtype=torch.int32)
+    taps = torch.zeros(out_size, ks, dtype=torch.float32)
+    lib.vqa_resample_table_tv(in_size, out_size, 0, out_size, C.cast(bounds.data_ptr(), C.POINTER(C.c_int32)),
+                              C.cast(taps.data_ptr(), C.POINTER(C.c_float)), C.byref(fma))
+    return bounds, taps, bool(fma.value)
+
+
 # ================================================================================================ Qwen2.5-VL
 def convert_qwen_state_dict(sd: Dict[str, torch.Tensor], cfg, device) -> Dict[str, torch.Tensor]:
     """HF `Qwen2_5_VLForConditionalGeneration` names -> the engine's fused bf16 layout:

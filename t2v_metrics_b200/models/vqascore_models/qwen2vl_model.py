@@ -1,10 +1,11 @@
-"""Qwen2.5-VL VQAScore plugin backed by the B200 engine (image inputs).
+"""Qwen2.5-VL VQAScore plugin backed by the B200 engine (images, video files and 4-D .npy frame stacks).
 
 Same plugin contract as the reference's `Qwen2VLModel` (t2v_metrics/models/vqascore_models/qwen2vl_model.py:93-301): class
 attributes, `forward(images, texts, question_template, answer_template, temperature) -> CPU fp32 Tensor[n]` with
 score = softmax(last-position logits / temperature)[first answer token]. The reference loops over samples and calls
-`generate(max_new_tokens=1)`; here the whole batch is ONE prefill in libvqa_b200.so and identical images are encoded once.
-Video inputs (decord / qwen_vl_utils frame sampling) are outside this engine's scope and raise.
+`generate(max_new_tokens=1)`; here the whole batch is ONE prefill in libvqa_b200.so and identical images or videos are encoded once.
+Videos follow qwen_vl_utils.fetch_video (frame sampling and sizing restated in qwen_utils); files are decoded by cv2 on the host
+instead of decord, and every frame's resize, normalisation and temporal pairing runs in one device kernel.
 """
 from __future__ import annotations
 
@@ -14,19 +15,15 @@ import torch
 
 from ...config import QWEN25VL_MODELS as _TABLE, Qwen25VLConfig
 from ...constants import HF_CACHE_DIR
-from .qwen_utils import qwen_image_to_patches, build_prompt_ids, default_question_template, default_answer_template
+from .qwen_utils import (QWEN_VL_UTILS_MAX_PIXELS, QWEN_VL_UTILS_MIN_PIXELS, REFERENCE_VIDEO_FPS, REFERENCE_VIDEO_MAX_PIXELS,
+                         VIDEO_EXTENSIONS, VIDEO_MIN_PIXELS, build_prompt_ids, decode_video_cv2,
+                         default_answer_template, default_question_template, qwen_image_to_patches, second_per_grid,
+                         video_max_pixels)
 from .vqa_model import VQAScoreModel
 
 QWEN2_VL_MODELS: Dict[str, dict] = {name: dict(model=dict(path=spec["weights"]), config=spec["config"]) for name, spec in _TABLE.items()}
 
 
-# Pixel bounds of the resize the reference applies BEFORE the HF processor: `process_vision_info` (qwen_vl_utils.vision_process.fetch_image)
-# calls smart_resize(h, w, factor=28, min_pixels=MIN_PIXELS, max_pixels=MAX_PIXELS) with MIN_PIXELS = 4 * 28 * 28 and
-# MAX_PIXELS = 16384 * 28 * 28, and the processor then runs with do_resize=False (reference qwen2vl_model.py:201-216), so the processor's own
-# 14*14*4*1280 ceiling never applies. qwen_vl_utils is an unpinned dependency that is not installed here: the two values are restated from
-# its source and exposed as constructor arguments (`min_pixels=`, `max_pixels=`) for other versions.
-QWEN_VL_UTILS_MIN_PIXELS = 4 * 28 * 28
-QWEN_VL_UTILS_MAX_PIXELS = 16384 * 28 * 28
 
 
 def _generation_config_penalty(checkpoint_path: str) -> float:
@@ -76,31 +73,65 @@ class Qwen2VLModel(VQAScoreModel):
         self.engine.load_state_dict(sd)
         self._state_dict = None
 
-    def load_images(self, image: List[str]):
-        """-> (patches fp32 [sum P, 1176] on the device, [(1, gh, gw), ...])"""
-        if any(p[-4:].lower() in (".mp4", ".avi", ".mov", ".mkv") for p in image):
-            raise NotImplementedError("video inputs are outside the B200 engine's hot-path scope")
-        # PIL decode on the host, everything else (smart_resize, PIL-exact bicubic, normalise, frame duplication, merge-order patch
-        # rows) in ONE device kernel -- bit-identical to qwen_utils.qwen_image_to_patches, the CPU path the reference runs per image
+    def load_images(self, image: List[str], fps=None):
+        """-> (patches fp32 [sum rows, 1176] on the device, [(t, gh, gw), ...], second_per_grid_ts per input, is_video per input), in
+        the order of `image`. Any mix of image files, 3-D .npy images, 4-D .npy frame stacks and video files (.mp4/.avi/.mov/.mkv);
+        `fps` applies to video files: None -> the model table's 8.0, a number, or "dynamic" (qwen_vl_utils' default FPS)."""
+        # Host work is decoding only (PIL for images, cv2 for files); smart_resize, the resize (PIL-exact for images and frame stacks,
+        # torchvision-exact for decoded files), normalisation, temporal pairing and merge-order patch rows run in one device kernel per
+        # kind -- bit-identical to qwen_utils.qwen_image_to_patches / qwen_video_to_patches, the CPU path the reference runs per sample.
         import numpy as np
         from PIL import Image
-        from ...engine import qwen_preprocess_u8
-        raw = []
-        for p in image:
-            if p.lower().endswith(".npy"):
-                # the reference's Qwen path takes the array as RGB, no channel flip (qwen2vl_model.py:146-153); 4-D arrays are frame stacks
+        from ... import _lib
+        from ...engine import qwen_preprocess_u8, qwen_video_preprocess_u8
+        fps = REFERENCE_VIDEO_FPS if fps is None else fps
+        stills, videos = [], []      # (position, uint8 tensor); videos: (position, frames, policy, min_pixels, max_pixels)
+        for i, p in enumerate(image):
+            low = p.lower()
+            if low.endswith(VIDEO_EXTENSIONS):
+                frames, _, _ = decode_video_cv2(p, fps)
+                videos.append((i, torch.from_numpy(frames), _lib.VQA_RESAMPLE_TORCHVISION, VIDEO_MIN_PIXELS,
+                               int(video_max_pixels(len(frames), REFERENCE_VIDEO_MAX_PIXELS))))
+            elif low.endswith(".npy"):
+                # the reference's Qwen path takes the array as RGB, no channel flip (qwen2vl_model.py:146-158)
                 arr = np.load(p)
-                if arr.ndim == 4:
-                    raise NotImplementedError("4-D .npy frame stacks are video inputs: outside the B200 engine's hot-path scope")
+                if arr.ndim == 4:         # a frame stack: a list of PIL frames through fetch_video's list branch
+                    arr = np.ascontiguousarray(arr.astype("uint8")[..., :3])
+                    if arr.shape[-1] != 3 or arr.shape[0] == 0:
+                        raise ValueError(f"Unexpected shape for NumPy array in {p}")
+                    videos.append((i, torch.from_numpy(arr), _lib.VQA_RESAMPLE_PIL, self.min_pixels, self.max_pixels))
+                    continue
                 if arr.ndim != 3:
                     raise ValueError(f"Unexpected shape for NumPy array in {p}")
                 arr = np.asarray(Image.fromarray(arr.astype("uint8"), "RGB"), dtype=np.uint8)
+                stills.append((i, torch.from_numpy(np.ascontiguousarray(arr))))
             else:
                 with Image.open(p) as im:
-                    arr = np.asarray(im.convert("RGB"), dtype=np.uint8)
-            raw.append(torch.from_numpy(np.ascontiguousarray(arr)))
-        return qwen_preprocess_u8(raw, self.engine.device, self.cfg.patch_size, self.cfg.temporal_patch_size, self.cfg.spatial_merge_size,
-                                  min_pixels=self.min_pixels, max_pixels=self.max_pixels)
+                    stills.append((i, torch.from_numpy(np.ascontiguousarray(np.asarray(im.convert("RGB"), dtype=np.uint8)))))
+        dev, cfg = self.engine.device, self.cfg
+        parts, order = [], []
+        if stills:
+            pt, g = qwen_preprocess_u8([t for _, t in stills], dev, cfg.patch_size, cfg.temporal_patch_size, cfg.spatial_merge_size,
+                                       min_pixels=self.min_pixels, max_pixels=self.max_pixels)
+            parts.append(pt)
+            order += [(i, grid, 1.0, False) for (i, _), grid in zip(stills, g)]
+        if videos:
+            pt, g = qwen_video_preprocess_u8([v[1] for v in videos], [v[2] for v in videos], dev, [v[3] for v in videos],
+                                             [v[4] for v in videos], cfg.patch_size, cfg.temporal_patch_size, cfg.spatial_merge_size)
+            parts.append(pt)
+            # what the reference's processor passes for every video on transformers 5.x (qwen_utils.PROCESSOR_FALLBACK_FPS)
+            order += [(v[0], grid, second_per_grid(cfg.temporal_patch_size), True) for v, grid in zip(videos, g)]
+        # rows must follow the order of `image`: stills come first, so reorder only when a video precedes an image
+        if [o[0] for o in order] != list(range(len(image))):
+            rows = [o[1][0] * o[1][1] * o[1][2] for o in order]
+            starts = [sum(rows[:k]) for k in range(len(rows))]
+            flat = torch.cat(parts)
+            by_pos = sorted(range(len(order)), key=lambda k: order[k][0])
+            patches = torch.cat([flat[starts[k]:starts[k] + rows[k]] for k in by_pos])
+            order = [order[k] for k in by_pos]
+        else:
+            patches = parts[0] if len(parts) == 1 else torch.cat(parts)
+        return patches, [o[1] for o in order], [o[2] for o in order], [o[3] for o in order]
 
     @torch.no_grad()
     def forward_with_trace(self, images: List[str], texts: List[str], fps=None, question_template: str = default_question_template,
@@ -146,7 +177,7 @@ class Qwen2VLModel(VQAScoreModel):
         answers = [answer_template.format(t) for t in texts]
         uniq: Dict[str, int] = {}
         index = [uniq.setdefault(p, len(uniq)) for p in images]
-        patches, grids = self.load_images(list(uniq.keys()))
+        patches, grids, spg, is_video = self.load_images(list(uniq.keys()), fps)
         unit = self.cfg.spatial_merge_size ** 2
         prompts, answer_ids = [], []
         cache = self.__dict__.setdefault("_prompt_cache", {})
@@ -154,7 +185,8 @@ class Qwen2VLModel(VQAScoreModel):
             cache.clear()
         for q, a, img in zip(questions, answers, index):
             t, gh, gw = grids[img]
-            prompts.append(build_prompt_ids(self.tokenizer, q, t * gh * gw // unit, self.cfg.image_token_id, cache))
+            token = self.cfg.video_token_id if is_video[img] else self.cfg.image_token_id
+            prompts.append(build_prompt_ids(self.tokenizer, q, t * gh * gw // unit, token, cache))
             ids = cache.get(("answer", a))
             if ids is None:
                 ids = cache[("answer", a)] = tuple(self.tokenizer.encode(a, add_special_tokens=False))
@@ -165,5 +197,6 @@ class Qwen2VLModel(VQAScoreModel):
             answer_ids.append(ids[0])
         self._last_answer_ids = list(answer_ids)
         probs = self.engine.score_prompts(patches, grids, prompts, answer_ids, image_of_sample=index, temperature=temperature,
-                                          repetition_penalty=self.repetition_penalty if repetition_penalty is None else repetition_penalty)
+                                          repetition_penalty=self.repetition_penalty if repetition_penalty is None else repetition_penalty,
+                                          second_per_grid_ts=spg if any(is_video) else None)
         return probs.float().cpu()

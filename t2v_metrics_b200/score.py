@@ -6,7 +6,8 @@ Differences, all above the drop-in boundary and result-preserving:
     image once. The reference loops `self.model.forward([image] * N, texts)` per image (score.py:104-106).
   * `batch_forward` scores a whole DataLoader batch per (visual, text) slot, as v3.0 did, instead of one pair at a time
     (v3.1 score.py:143-153).
-  * video inputs (the cv2 concat path, score.py:72-98) are CPU pre-processing outside this engine's scope and raise.
+  * video paths go to plugins with `video_mode == "direct"` (Qwen2.5-VL), which sample, resize and encode the frames themselves.
+    The cv2 frame-concatenation path of `video_mode == "concat"` plugins (reference score.py:72-98) is not built and raises.
 """
 from typing import List, Optional, TypedDict, Union
 
@@ -49,9 +50,10 @@ class Score(nn.Module):
             images = [images]
         if isinstance(texts, str):
             texts = [texts]
-        if any(isinstance(img, str) and img[-4:].lower() in VIDEO_EXTENSIONS for img in images):
+        if any(isinstance(img, str) and img[-4:].lower() in VIDEO_EXTENSIONS for img in images) and \
+                getattr(self.model, "video_mode", None) != "direct":
             raise NotImplementedError("video inputs (frame extraction + concat, reference score.py:72-98) are outside the "
-                                      "B200 engine's hot-path scope; pass image files")
+                                      "B200 engine's hot-path scope for this model; pass image files or use a direct-video model")
         m, n = len(images), len(texts)
         import torch.distributed as dist
         world = dist.get_world_size() if (self.shard_over_images and dist.is_available() and dist.is_initialized()) else 1
@@ -77,22 +79,28 @@ class Score(nn.Module):
         return local.view(m, n).to(self.device)
 
     def batch_forward(self, dataset: List[ImageTextDict], batch_size: int = 16, num_frames: int = 4, **kwargs) -> torch.Tensor:
-        """[num_samples, num_visuals, num_texts] scores for a dataset of {'images': [...], 'texts': [...]} items."""
+        """[num_samples, num_visuals, num_texts] scores for a dataset of {'images': [...], 'texts': [...]} items, or, for models with
+        `video_mode == "direct"`, of {'videos': [...], 'texts': [...]} items, scored exactly like images (the plugin takes the paths).
+        The reference's own video branch calls `self.forward(videos=...)`, a keyword its forward does not accept; here video datasets
+        go through the same per-slot plugin calls as images instead."""
         from torch.utils.data import DataLoader
         num_samples = len(dataset)
+        key = 'images'
         if "videos" in dataset[0]:
-            raise NotImplementedError("video datasets are outside the B200 engine's hot-path scope")
-        num_visuals = len(dataset[0]['images'])
+            if getattr(self.model, "video_mode", None) != "direct":
+                raise NotImplementedError("video datasets need a model with video_mode 'direct'; the concat path is not built")
+            key = 'videos'
+        num_visuals = len(dataset[0][key])
         num_texts = len(dataset[0]['texts'])
         scores = torch.zeros(num_samples, num_visuals, num_texts).to(self.device)
         dataloader = DataLoader(dataset, batch_size=batch_size, shuffle=False)
         counter = 0
         for batch_idx, batch in enumerate(dataloader):
-            cur = len(batch['images'][0])
-            assert len(batch['images']) == num_visuals and len(batch['texts']) == num_texts
+            cur = len(batch[key][0])
+            assert len(batch[key]) == num_visuals and len(batch['texts']) == num_texts
             for vis_idx in range(num_visuals):
                 for text_idx in range(num_texts):
                     scores[counter:counter + cur, vis_idx, text_idx] = self.model.forward(
-                        list(batch['images'][vis_idx]), list(batch['texts'][text_idx]), **kwargs).to(self.device)
+                        list(batch[key][vis_idx]), list(batch['texts'][text_idx]), **kwargs).to(self.device)
             counter += cur
         return scores
